@@ -51,7 +51,42 @@ def parse():
     p.add_argument("--no-prefetch", action="store_true",
                    help="do not announce the next batch's ids one step ahead (default: the public prefetch API, the reference's "
                         "pulling(): the next batch's pull + plan run beside this step's dense all-reduce / optimizer)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="write what the last device-timed step computed as DIR/<name>.npy (float32, rank 0): its loss, "
+                        "the dense parameters after its update and the embedding rows of its batch read back after it")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        p.error("--dump-outputs covers --impl ours")
+    return a
+
+
+DUMP_PARAMS = 4 << 20           # floats of dense parameters, at most (16 MB)
+DUMP_ROWS_BYTES = 32 << 20      # bytes of embedding rows, at most: a dump stays under 64 MB
+
+
+def _sample_rows(torch, t, n, seed):
+    """``t`` if it has at most ``n`` rows, else ``n`` of its rows (in order, with repeats) picked by a fixed seed"""
+    if t.shape[0] <= n:
+        return t
+    g = torch.Generator(device="cpu").manual_seed(seed)
+    idx = torch.randint(t.shape[0], (n,), generator=g).sort().values
+    return t[idx.to(t.device)]
+
+
+def dump_outputs(torch, model, loss, ids):
+    """What a training step computed, as float32 host arrays: ``loss`` (what ``step`` returns), the dense parameters
+    after its update (flat, in the model's order; replicated small tables included) and the server-side embedding
+    rows of its batch ``ids`` read back by a stateless pull ([batch, io_stride], the model's activation layout;
+    columns no server table feeds are 0). Larger outputs are cut to a seeded sample of rows."""
+    dense = model.theta if hasattr(model, "theta") else torch.cat([p.detach().reshape(-1) for p in model.dense_parameters()])
+    out = {"loss": loss.detach().reshape(1), "dense_params": _sample_rows(torch, dense, DUMP_PARAMS, 1)}
+    if model.sparse is not None:
+        rows = torch.zeros((ids.shape[0], model.sparse.io_stride), dtype=torch.float32, device=ids.device)
+        rows = model.sparse.group.pull(ids, out=rows)
+        out["embedding_rows"] = _sample_rows(torch, rows, max(1, DUMP_ROWS_BYTES // (4 * rows.shape[1])), 2)
+    return {k: v.float().cpu().numpy() for k, v in out.items()}
 
 
 class ClockSampler:
@@ -289,6 +324,7 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms = float(t[0])
     ctx.backend.engine.check()
+    dumped = dump_outputs(torch, model, loss, devb[(a.warmup + a.steps - 1) % a.pool][0]) if a.dump_outputs else None
 
     # ---------------- end-to-end through the public pipeline API: pinned H2D in, loss D2H out, every step
     pipe = trainer.make_pipeline(a.batch, len(vocab), 13)
@@ -354,6 +390,11 @@ def main():
                                          "nvlink_rows_pulled", "nvlink_rows_pushed", "plans")},
         }
         print(json.dumps(line))
+        if dumped is not None:
+            import numpy as np
+            os.makedirs(a.dump_outputs, exist_ok=True)
+            for name, arr in dumped.items():
+                np.save(os.path.join(a.dump_outputs, name + ".npy"), arr)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()

@@ -6,9 +6,10 @@ Two shared libraries with a C ABI (the "narrow waist", like the reference's
 * ``lib/libexb_core.so``  -- C++17 CPU engine + checkpoint IO (g++)
 * ``lib/libexb_cuda.so``  -- sm_100a kernels + CUDA runtime glue (nvcc)
 
-The libraries are built *in tree* so that a ``gpurun`` snapshot carries them to the
-GPU box; a content hash of sources+flags is stored next to each ``.so`` so an
-up-to-date library is loaded without invoking the compiler.
+The libraries are built *in tree*, so a copy of the built tree carries them to
+another machine; a content hash of sources+flags is stored next to each ``.so`` so an
+up-to-date library is loaded without invoking the compiler and without writing to
+the tree (which may be read-only after the build).
 """
 import concurrent.futures
 import hashlib
@@ -91,12 +92,25 @@ class _BuildLock:
         self.fh.close()
 
 
+def _core_deps():
+    return _sources("core", (".cpp",)) + _sources("core", (".h",))
+
+
+def _cuda_deps():
+    return _sources("cuda", (".cu",)) + _sources("cuda", (".cuh", ".h")) + _sources("core", (".h",))
+
+
+# An up-to-date library is returned before the lock is taken: the lock file is opened for writing.
 def build_core(force=False, verbose=False):
+    if not force and _stamp_ok(core_lib_path(), _hash(_core_deps(), CXX_FLAGS)):
+        return core_lib_path()
     with _BuildLock():
         return _build_core(force, verbose)
 
 
 def build_cuda(force=False, verbose=False):
+    if not force and _stamp_ok(cuda_lib_path(), _hash(_cuda_deps(), NVCC_FLAGS)):
+        return cuda_lib_path()
     with _BuildLock():
         return _build_cuda(force, verbose)
 
@@ -104,7 +118,7 @@ def build_cuda(force=False, verbose=False):
 def _build_core(force=False, verbose=False):
     os.makedirs(_LIB, exist_ok=True)
     srcs = _sources("core", (".cpp",))
-    deps = srcs + _sources("core", (".h",))
+    deps = _core_deps()
     digest = _hash(deps, CXX_FLAGS)
     lib = core_lib_path()
     if not force and _stamp_ok(lib, digest):
@@ -124,7 +138,7 @@ def _build_core(force=False, verbose=False):
 def _build_cuda(force=False, verbose=False):
     os.makedirs(_OBJ, exist_ok=True)
     srcs = _sources("cuda", (".cu",))
-    deps = srcs + _sources("cuda", (".cuh", ".h")) + _sources("core", (".h",))
+    deps = _cuda_deps()
     digest = _hash(deps, NVCC_FLAGS)
     lib = cuda_lib_path()
     if not force and _stamp_ok(lib, digest):

@@ -198,6 +198,7 @@ class _Pipeline:
         self.done = [torch.cuda.Event() for _ in range(n)]
         self.k = 0            # batches submitted
         self.trained = 0      # batches trained
+        self.waited = -1      # last batch whose copy the compute stream waited for in submit()
         self.h2d_bytes = batch * num_sparse * 8 + batch * num_dense * 4 + batch * 4
         self.d2h_bytes = 4
 
@@ -235,11 +236,12 @@ class _Pipeline:
         self.k = k + 1
         if not self.lookahead:
             self._train(k, None)
-        elif k >= 1:
+        elif self.trained < k:        # right after flush() batch k-1 is trained already; the next submit trains batch k
             cur = torch.cuda.current_stream(self.t.device)
             cur.wait_event(self.copied[i])                    # the plan kernel of batch k reads its ids
-            # batch k-1's copy was waited for by the previous submit (as "next ids") -- except for the very first one
-            self._train(k - 1, self.dev[i]["ids"], copied_waited=k >= 2)
+            # batch k-1's copy was waited for by the previous submit (as "next ids") -- if that one trained a batch
+            self._train(k - 1, self.dev[i]["ids"], copied_waited=self.waited == k - 1)
+            self.waited = k
 
     def flush(self):
         while self.trained < self.k:

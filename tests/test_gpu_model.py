@@ -68,6 +68,38 @@ def test_graph_matches_eager(cuda_context):
         assert abs(a - b) < 1e-3, res
 
 
+class _CountingTrainer:
+    """a trainer with next-batch prefetch that records which batch every step trains (the batch number is its ids)"""
+    supports_prefetch = want_prefetch = True
+
+    def __init__(self, device):
+        self.device, self.trained = device, []
+
+    def step(self, ids, dense, labels, next_ids=None, stable=False):
+        self.trained.append(int(ids[0, 0]))
+        return labels.sum()
+
+
+def test_pipeline_trains_every_batch_once(cuda_context):
+    """the one-batch-ahead input pipeline trains each submitted batch exactly once, also when last_loss() drains it
+    between two runs of submits"""
+    from openembedding_b200.models.trainer import _Pipeline
+    tr = _CountingTrainer(torch.device("cuda", torch.cuda.current_device()))
+    pipe = _Pipeline(tr, 4, 2, 1)
+
+    def submit(k):
+        pipe.submit(torch.full((4, 2), k, dtype=torch.int64).pin_memory(), torch.zeros(4, 1).pin_memory(),
+                    torch.full((4,), float(k)).pin_memory())
+
+    for k in range(5):
+        submit(k)
+    assert pipe.last_loss() == 4 * 4
+    for k in range(5, 12):
+        submit(k)
+    assert pipe.last_loss() == 4 * 11
+    assert tr.trained == list(range(12))
+
+
 def test_api_embedding_checkpoint_roundtrip(cuda_context):
     import openembedding_b200.torch as embed
     from openembedding_b200.context import get_context
